@@ -29,7 +29,11 @@ Further objects on the same JSON line (N=1 unless noted; each can be switched of
   config1_filmtrust  BASELINE config 1: the recorded reference run replayed through the drop-in class
   zipf_contended     the fused epoch on Zipf-distributed items
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the timed path computed, as of its last timed step, to DIR/<name>.npy: the tables P and Q
+and the step's loss terms.  A table larger than DUMP_TABLE_BYTES is cut to a fixed, seeded sample of its rows.  The inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -53,6 +57,7 @@ METRIC = 'BPR triples/sec at d=64'
 LIGHTGCN_MULTI_SCHEME = 'user'        # 'cols' once its N>1 numbers are in (QREC_LGCN_SCHEME overrides)
 MULTI_GPU_DEFAULTS = {'qsync': 'auto', 'lightgcn_multi': True, 'parity_multi': True}     # validated at N=2 (profiles/r2/multi_n2)
 WORKLOAD = 'BPR synthetic 1M users x 100K items x 50M interactions, d=64, fp32, user-major (reference) order'
+DUMP_TABLE_BYTES = 28 << 20          # per table: P and Q together stay under 64 MB in float32 and in float64
 
 
 def measured_hbm_peak():
@@ -121,6 +126,21 @@ class ClockSampler(object):
                 'samples': len(sm)}
 
 
+def dump_rows(n, row_bytes):
+    """Rows of an n-row table that --dump-outputs writes: all of them, or, above DUMP_TABLE_BYTES, the same seeded
+    sample on every run."""
+    if n * row_bytes <= DUMP_TABLE_BYTES:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_TABLE_BYTES // row_bytes, replace=False))
+
+
+def dump_outputs(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + '.npy'), np.ascontiguousarray(a))
+
+
 # ---------------------------------------------------------------------------------------------
 # reference arm / cpu baseline: the oracle port of the reference's numpy loop on host cores
 # ---------------------------------------------------------------------------------------------
@@ -168,9 +188,12 @@ def run_reference(args):
     t0 = time.perf_counter()
     for k in range(args.steps):
         s = slice((args.warmup + k) * sample, (args.warmup + k + 1) * sample)
-        c_oracle.bpr_sgd_sequential(P, Q, u[s], i[s], j[s], LR, REG_U, REG_I)
+        loss = c_oracle.bpr_sgd_sequential(P, Q, u[s], i[s], j[s], LR, REG_U, REG_I)
     dt = time.perf_counter() - t0
     value = sample * args.steps / dt
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {'P': P[dump_rows(len(P), P[0].nbytes)], 'Q': Q[dump_rows(len(Q), Q[0].nbytes)],
+                                         'loss': np.array([loss])})
     desc = ('%d user-major triples per step (fresh users each step) of the same workload; float64 C port (oracle/bpr_ref.c) of '
             'model/ranking/BPR.py:45-53; the Python reference itself cannot travel to the GPU box '
             '(measured here: ~95 K triples/s); serial dependency chain => 1 thread of %d' % (sample, os.cpu_count() or 0))
@@ -799,6 +822,10 @@ def run_ours(args):
     assert np.isfinite(epoch_loss), 'loss is not finite'
     total_triples = n_local * world * args.steps
     value = total_triples / (elapsed_ms * 1e-3)
+    if args.dump_outputs and rank == 0:       # N>1: rank 0's user shard of P; Q is the same on every rank after drain()
+        p_rows = torch.from_numpy(dump_rows(users_local, P[0].nbytes)).to(dev)
+        dump_outputs(args.dump_outputs, {'P': P[p_rows].cpu().numpy(), 'Q': Q.cpu().numpy()[dump_rows(NUM_ITEMS, Q[0].nbytes)],
+                                         'loss': final})       # sum(-ln sigmoid), |P|^2, |Q|^2 of the last timed epoch
 
     # ------------------------------------------------------------------ the same epoch, shuffled order
     perm = torch.randperm(n_local, device=dev, generator=g)
@@ -1107,6 +1134,8 @@ def main():
     ap.add_argument('--no-extras', action='store_true', help='skip the FilmTrust (config 1) and Zipf sections')
     ap.add_argument('--no-roofs', action='store_true', help='skip the row-op microbenchmark and the HBM-bound configuration')
     ap.add_argument('--no-parity', action='store_true', help='skip the full-epoch parity check against the sequential oracle')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the tables and the loss of the last timed step to DIR/<name>.npy '
+                    '(tables above %d MiB: a fixed seeded sample of their rows)' % (DUMP_TABLE_BYTES >> 20))
     args = ap.parse_args()
     assert args.warmup >= 0 and args.steps >= 1
     if args.impl == 'reference':

@@ -1,8 +1,8 @@
 #!/usr/bin/env python
-"""Golden-vector generator: runs the UNMODIFIED reference (Coder-Yu/QRec, mounted
-read-only at /root/reference) in this container and records what the hot path
-consumed and produced.  TEST INFRASTRUCTURE ONLY -- nothing in the product path
-imports this file; the GPU box never runs it (there is no /root/reference there).
+"""Golden-vector generator: runs the UNMODIFIED reference (a Coder-Yu/QRec checkout, found at
+$QREC_REFERENCE_DIR) and records what the hot path consumed and produced.  TEST INFRASTRUCTURE
+ONLY -- nothing in the product path imports this file, and no test needs the reference checkout:
+the tests read only what this file wrote under tests/golden/.
 
 What is exercised (reference file:line):
   * QRec.__init__            QRec.py:8-47        load FilmTrust, `-ap 0.2 -b 1` split
@@ -18,12 +18,15 @@ What is exercised (reference file:line):
     (pointwise sequential SGD; §8 f-4), with the per-epoch shuffle of isConverged and the
     MAE / RMSE of evalRatings (base/recommender.py:95-125, util/measure.py)
   * SBPR.initModel / next_batch   model/ranking/SBPR.py:12-29, 69-101 (social-feedback sets, minibatch sampler)
+  * the host-side modules under differential test (gen_differential) and TBPR / SBPR on the inputs of
+    their CPU tests (gen_social)
 
 `tensorflow` and `mkl` are absent from this image; both are stubbed with empty
 modules because the reference imports them at module level (model/ranking/BPR.py:7,
 QRec.py:6).  The numpy path never calls into either.
 
-Usage:  python oracle/gen_golden.py [bpr] [mf] [sbpr]   (default: all sections; writes tests/golden/*.npz)
+Usage:  QREC_REFERENCE_DIR=<QRec checkout> python oracle/gen_golden.py [bpr] [mf] [sbpr] [differential] [social]
+        (default: all sections; writes tests/golden/*.npz, *.json.xz, *.txt.xz; needs the built package for `social`)
 """
 import os
 import sys
@@ -35,7 +38,7 @@ import io
 
 import numpy as np
 
-REF = '/root/reference'
+REF = os.environ.get('QREC_REFERENCE_DIR', '')
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OUT = os.path.join(REPO, 'tests', 'golden')
 
@@ -389,8 +392,226 @@ def gen_sbpr():
     print('sbpr: %d relations, %d users with social feedback, 8 batches of 512' % (len(relation), int((fp_sizes > 0).sum())))
 
 
+def _quiet(fn, *a, **kw):
+    with contextlib.redirect_stdout(io.StringIO()):
+        return fn(*a, **kw)
+
+
+def gen_differential():
+    """Inputs and outputs of the reference's host-side surface for tests/test_differential_reference.py, plus
+    FilmTrust's ratings file itself (tests/golden/filmtrust_ratings.txt.xz, read by the loader tests).  The tests
+    draw the same seeded random inputs again, so only the reference's outputs are stored:
+      * util/config.py OptionConf / ModelConf   on random option strings and on every config/*.conf
+      * util/measure.py rankingMeasure / ratingMeasure, util/qmath.py find_k_largest / sigmoid
+      * data/rating.py Rating under four evaluation setups, util/dataSplit.py dataSplit / crossValidation
+      * util/io.py loadDataSet on FilmTrust (digests: the full lists are 35K records each) and the id space of
+        Rating over it
+      * base/iterativeRecommender.py isConverged + base/recommender.py evalRanking, and
+        base/deepRecommender.py next_batch_pairwise / next_batch_pointwise on random interaction lists (digests)"""
+    import importlib
+    import lzma
+    from oracle import golden_json
+    M = {n: importlib.import_module(n) for n in ('util.config', 'util.measure', 'util.qmath', 'util.io', 'util.dataSplit',
+                                                 'data.rating', 'base.iterativeRecommender', 'base.deepRecommender')}
+    RConf = M['util.config'].ModelConf
+
+    def conf_of(config):
+        c = RConf.__new__(RConf)
+        c.config = dict(config)
+        return c
+    rec = {}
+
+    rng = random.Random(0)
+    vocab = ['on', 'off', '-a', '-b', '--c', '-topN', '-1', '-12', '-0.5', '5', '10,20', 'x', '0.1', '-tf', '', '-n_layer', '2']
+    rows = []
+    for _ in range(3000):
+        s = ' '.join(rng.choice(vocab) for _ in range(rng.randint(1, 8)))
+        if rng.random() < 0.2:
+            s = ' ' + s + ' '
+        o = M['util.config'].OptionConf(s)
+        rows.append((o.options, o.isMainOn(), o.line))
+    rec['option_conf'] = rows
+
+    cdir = os.path.join(REF, 'config')
+    rec['model_conf'] = [(name, open(os.path.join(cdir, name)).read(), RConf(os.path.join(cdir, name)).config)
+                         for name in sorted(os.listdir(cdir))]
+    with open('bad.conf', 'w') as f:
+        f.write('a=1\nnot a pair\nb=2=3\n\nc=x y\n')
+    rec['model_conf_bad'] = RConf('bad.conf').config
+
+    R = M['util.measure'].Measure
+    rng = random.Random(1)
+    items = ['i%d' % k for k in range(60)]
+    cases = []
+    for _ in range(200):
+        users = ['u%d' % k for k in range(rng.randint(1, 12))]
+        origin = {u: {it: 1.0 for it in rng.sample(items, rng.randint(1, 15))} for u in users}
+        res = {u: [(it, rng.random()) for it in rng.sample(items, 20)] for u in users}
+        tops = sorted(rng.sample([1, 3, 5, 10, 20], rng.randint(1, 3)))
+        cases.append(R.rankingMeasure(origin, res, tops))
+    rows = [['u', 'i', rng.random() * 5, rng.random() * 5] for _ in range(50)]
+    rec['ranking_measure'] = cases
+    rec['rating_measure'] = (R.ratingMeasure(rows), R.ratingMeasure([]))
+
+    F = M['util.qmath'].find_k_largest
+    rng = np.random.default_rng(2)
+    trials = []
+    for trial in range(120):
+        n, K = int(rng.integers(3, 300)), int(rng.integers(1, 15))
+        s = rng.standard_normal(n).round(1 if trial % 3 == 0 else 7)
+        s[rng.integers(0, n, n // 5)] = 0.0                       # rated items are overwritten with 0
+        ids, vals = F(K, s.copy())
+        trials.append((list(ids), list(vals)))
+    rec['find_k_largest'] = trials
+    rec['sigmoid_0.3'] = M['util.qmath'].sigmoid(0.3)
+
+    rng = random.Random(3)
+    runs = []
+    for ev in ('-ap 0.2', '-ap 0.2 -b 1', '-cold 2', '-val 0.25'):
+        train = [['u%d' % rng.randint(0, 30), 'i%d' % rng.randint(0, 40), float(rng.randint(1, 5))] for _ in range(400)]
+        test = [['u%d' % rng.randint(0, 35), 'i%d' % rng.randint(0, 45), float(rng.randint(1, 5))] for _ in range(120)]
+        random.seed(11)
+        d = M['data.rating'].Rating(conf_of({'ratings': 'x', 'evaluation.setup': ev}), [r[:] for r in train], [r[:] for r in test])
+        u0 = next(iter(d.user))
+        out = {a: getattr(d, a) for a in ('user', 'item', 'id2user', 'id2item', 'userMeans', 'itemMeans', 'globalMean',
+                                          'rScale', 'trainingData', 'testData')}
+        out.update(trainSet_u=dict(d.trainSet_u), testSet_u=dict(d.testSet_u), trainSet_i=dict(d.trainSet_i),
+                   testSet_i=dict(d.testSet_i), trainingSize=d.trainingSize(), testSize=d.testSize(), u0=u0,
+                   userRated=d.userRated(u0), row=d.row(u0))
+        runs.append(out)
+    rec['rating'] = runs
+
+    RS = M['util.dataSplit'].DataSplit
+    rng = random.Random(5)
+    data = [['u%d' % rng.randint(0, 9), 'i%d' % rng.randint(0, 9), float(rng.randint(0, 1))] for _ in range(300)]
+    split = []
+    for ratio, binar in ((0.2, False), (0.2, True), (1.5, False), (0.0, True)):
+        random.seed(7)
+        split.append((RS.dataSplit(data, test_ratio=ratio, binarized=binar), random.getstate()))
+    cv = [list(RS.crossValidation(data, k, binarized=binar)) for k, binar in ((5, False), (3, True), (1, False), (11, False))]
+    rec['data_split'] = (split, cv)
+
+    path = os.path.join(REF, 'dataset', 'FilmTrust', 'ratings.txt')
+    loads = []
+    for setup, kw in (('-columns 0 1 2', {}), ('-columns 0 1 2', {'binarized': True, 'threshold': 3.0}),
+                      ('-columns 1 0', {}), ('-columns 0 1 2 -header', {'bTest': True})):
+        b = _quiet(M['util.io'].FileIO.loadDataSet, conf_of({'ratings.setup': setup}), path, **kw)
+        loads.append((len(b), b[:5], golden_json.digest(b)))
+    rec['load_filmtrust'] = loads
+    rc = conf_of({'ratings.setup': '-columns 0 1 2', 'evaluation.setup': '-ap 0.2 -b 1'})
+    recs = _quiet(M['util.io'].FileIO.loadDataSet, rc, path, binarized=True, threshold=1.0)
+    d = M['data.rating'].Rating(rc, recs, [])
+    rec['table_filmtrust'] = dict(n=len(recs), user_names=[d.id2user[k] for k in range(len(d.user))],
+                                  item_names=[d.id2item[k] for k in range(len(d.item))],
+                                  u_digest=golden_json.digest([d.user[r[0]] for r in recs]),
+                                  i_digest=golden_json.digest([d.item[r[1]] for r in recs]))
+
+    rng = random.Random(9)
+    conf_text = ('ratings=x\nratings.setup=-columns 0 1 2\nmodel.name=BPR\nevaluation.setup=-ap 0.2 -b 1\n'
+                 'item.ranking=on -topN 5,10\nnum.factors=8\nnum.max.epoch=3\nlearnRate=-init 0.01 -max 0.0105\n'
+                 'reg.lambda=-u 0.001 -i 0.001 -b 0.2 -s 0.2\noutput.setup=on -dir ./results/\n')
+    train = [['u%d' % rng.randint(0, 40), 'i%d' % rng.randint(0, 60), 1.0] for _ in range(900)]
+    test = [['u%d' % rng.randint(0, 45), 'i%d' % rng.randint(0, 60), 1.0] for _ in range(200)]
+    with open('eval.conf', 'w') as f:
+        f.write(conf_text)
+    m = M['base.iterativeRecommender'].IterativeRecommender(RConf('eval.conf'), [r[:] for r in train], [r[:] for r in test])
+    with contextlib.redirect_stdout(io.StringIO()):
+        m.readConfiguration()
+        m.initializing_log()
+        np.random.seed(4)
+        m.initModel()
+        random.seed(21)
+        conv = []
+        for epoch, loss in enumerate([100.0, 90.0, 95.0, 94.9995], 1):
+            m.loss = loss
+            conv.append((m.isConverged(epoch), m.lRate))
+        m.evalRanking()
+    rec['eval_ranking'] = (conv, m.recOutput, m.measure, random.getstate(), [r[:] for r in m.data.trainingData])
+
+    batches = {}
+    for seed in (0, 7, 2024):
+        rng = random.Random(seed)
+        conf_text = ('ratings=x\nratings.setup=-columns 0 1 2\nmodel.name=LightGCN\nevaluation.setup=-ap 0.2\n'
+                     'item.ranking=on -topN 10\nnum.factors=8\nnum.max.epoch=1\nbatch_size=128\n'
+                     'learnRate=-init 0.01 -max 1\nreg.lambda=-u 0.001 -i 0.001 -b 0.2 -s 0.2\noutput.setup=off -dir ./results/\n')
+        train = [['u%d' % rng.randint(0, 50), 'i%d' % rng.randint(0, 80), float(rng.randint(1, 5))] for _ in range(1000)]
+        with open('batch.conf', 'w') as f:
+            f.write(conf_text)
+        m = M['base.deepRecommender'].DeepRecommender(RConf('batch.conf'), [r[:] for r in train], [])
+        _quiet(m.readConfiguration)
+        random.seed(seed)
+        pair = [tuple(np.asarray(x).tolist() for x in batch) for batch in m.next_batch_pairwise()]
+        point = [tuple(np.asarray(x).tolist() for x in batch) for batch in m.next_batch_pointwise()]
+        batches[seed] = (len(pair), golden_json.digest(pair), golden_json.digest(point),
+                         golden_json.digest([r[:] for r in m.data.trainingData]), random.getstate())
+    rec['minibatch'] = batches
+
+    golden_json.save(os.path.join(OUT, 'differential_reference.json.xz'), rec)
+    with open(path, 'rb') as f, lzma.open(os.path.join(OUT, 'filmtrust_ratings.txt.xz'), 'wb', preset=9) as g:
+        g.write(f.read())
+    print('differential: %d option strings, %d config files, %d ranking cases' % (
+        len(rec['option_conf']), len(rec['model_conf']), len(rec['ranking_measure'])))
+
+
+TBPR_ROWS = np.arange(0, 310, 5)          # every 5th row of both tables is stored whole (P has 310 rows)
+
+
+def gen_social():
+    """model/ranking/TBPR.py (whole numpy run) and model/ranking/SBPR.py:12-29,69-101 (item sets + sampler) of the
+    UNMODIFIED reference classes on the inputs tests/test_tbpr_cpu.py and tests/test_sbpr_cpu.py build (a FilmTrust
+    training prefix + a synthetic trust network).  TBPR iterates a Python set of item names (TBPR.py:122), so its
+    stream depends on the string-hash seed: main() runs every section with PYTHONHASHSEED=0 and the TBPR test replays
+    the drop-in under the same seed."""
+    import importlib
+    from oracle import golden_json
+    sys.path.insert(0, os.path.join(REPO, 'tests'))
+    import test_tbpr_cpu
+    import test_sbpr_cpu
+    g = np.load(os.path.join(OUT, 'bpr_filmtrust_seed0.npz'))
+    RConf = importlib.import_module('util.config').ModelConf
+
+    R = importlib.import_module('model.ranking.TBPR').TBPR
+    train, test, rel = test_tbpr_cpu._data(g)
+    with open('tbpr.conf', 'w') as f:
+        f.write(test_tbpr_cpu.CONF)
+    random.seed(11); np.random.seed(11)
+    ref = R(RConf('tbpr.conf'), [list(r) for r in train], [list(r) for r in test], [list(r) for r in rel])
+    losses = []
+    orig = R.isConverged
+    R.isConverged = lambda self, epoch: (losses.append((self.loss, self.lRate)), orig(self, epoch))[1]
+    try:
+        measure = _quiet(ref.execute)
+    finally:
+        R.isConverged = orig
+    np.savez_compressed(os.path.join(OUT, 'tbpr_reference_hashseed0.npz'),
+                        theta=np.array(ref.theta), t_s=np.array(ref.t_s), t_w=np.array(ref.t_w),
+                        loss=np.array([l[0] for l in losses]), lrate=np.array([l[1] for l in losses]),
+                        rows=TBPR_ROWS, P_rows=ref.P[TBPR_ROWS], Q_rows=ref.Q[TBPR_ROWS], P_abs_row_sums=np.abs(ref.P).sum(1),
+                        Q_abs_row_sums=np.abs(ref.Q).sum(1), measure=np.array([x.strip() for x in measure]))
+
+    R = importlib.import_module('model.ranking.SBPR').SBPR
+    train, test, rel = test_tbpr_cpu._data(g, 3000)
+    with open('sbpr.conf', 'w') as f:
+        f.write(test_sbpr_cpu.CONF)
+    np.random.seed(1)
+    ref = R(RConf('sbpr.conf'), [list(r) for r in train], [list(r) for r in test], [list(r) for r in rel])
+    _quiet(ref.readConfiguration)
+    _quiet(ref.initModel)
+    ref.batch_size = 700
+    random.seed(77)
+    batches = [tuple(list(x) for x in b) for b in ref.next_batch()]
+    golden_json.save(os.path.join(OUT, 'sbpr_reference_sampler.json.xz'), dict(
+        positive={u: dict(v) for u, v in ref.PositiveSet.items() if v},
+        fp={u: dict(v) for u, v in ref.FPSet.items()},
+        batches=batches, state=random.getstate()))
+    print('social: TBPR losses %s, SBPR %d batches' % ([l[0] for l in losses], len(batches)))
+
+
 def main():
-    what = set(sys.argv[1:]) or {'bpr', 'mf', 'sbpr'}
+    if os.environ.get('PYTHONHASHSEED') != '0':      # gen_social's TBPR stream depends on the string-hash seed
+        os.execve(sys.executable, [sys.executable] + sys.argv, dict(os.environ, PYTHONHASHSEED='0'))
+    what = set(sys.argv[1:]) or {'bpr', 'mf', 'sbpr', 'differential', 'social'}
+    sys.path.insert(0, REPO)
     _enter_workdir()
     if 'bpr' in what:
         gen_bpr()
@@ -398,6 +619,10 @@ def main():
         gen_mf()
     if 'sbpr' in what:
         gen_sbpr()
+    if 'differential' in what:
+        gen_differential()
+    if 'social' in what:
+        gen_social()
 
 
 if __name__ == '__main__':

@@ -89,14 +89,17 @@ def test_measure_definitions():
     assert Measure.ratingMeasure([['u', 'i', 3.0, 2.0], ['u', 'j', 1.0, 2.0]]) == ['MAE:1.0\n', 'RMSE:1.0\n']
 
 
-@pytest.mark.skipif(not os.path.exists('/root/reference/dataset/FilmTrust/ratings.txt'),
-                    reason='reference dataset only exists in the build container')
 def test_loader_and_split_reproduce_reference_split(golden_bpr, tmp_path, monkeypatch):
-    """QRec.__init__ (QRec.py:8-47): loadDataSet + seeded -ap split give the recorded training
-    list and leave Python's MT19937 in the recorded state."""
+    """QRec.__init__ (QRec.py:8-47): loadDataSet + seeded -ap split of FilmTrust's ratings file
+    (tests/golden/filmtrust_ratings.txt.xz) give the recorded training list and leave Python's MT19937
+    in the recorded state."""
+    import lzma
+    from conftest import GOLDEN
     from qrec_b200.QRec import QRec
     monkeypatch.chdir(tmp_path)
-    os.symlink('/root/reference/dataset', tmp_path / 'dataset')
+    os.makedirs('dataset/FilmTrust')
+    with lzma.open(os.path.join(GOLDEN, 'filmtrust_ratings.txt.xz')) as f:
+        (tmp_path / 'dataset' / 'FilmTrust' / 'ratings.txt').write_bytes(f.read())
     random.seed(0)
     q = QRec(_conf(str(golden_bpr['conf'])))
     assert [r[0] for r in q.trainingData] == golden_bpr['train_users'].tolist()

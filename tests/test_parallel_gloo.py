@@ -426,7 +426,7 @@ def _exit_decision_worker(rank, world, port, out):
         dist.destroy_process_group()
 
 
-def test_exit_decision_after_graph_capture_is_collective_world2():
+def test_exit_decision_after_graph_capture_is_collective_world2(monkeypatch):
     """bench.py / the tools end through parallel.finish_process() when ANY rank holds a captured NCCL graph: a rank
     deciding on its own would leave the others in the barrier."""
     port = 36300 + os.getpid() % 2000
@@ -434,7 +434,11 @@ def test_exit_decision_after_graph_capture_is_collective_world2():
     out = mgr.dict()
     mp.spawn(_exit_decision_worker, args=(2, port, out), nprocs=2, join=True)
     assert dict(out) == {0: 1, 1: 1}
-    assert parallel.any_rank_captured_graphs() is False          # no process group: this process's own count
+    # no process group: this process's own count (pinned here: GPU tests earlier in the session may have captured graphs)
+    monkeypatch.setattr(parallel, '_CAPTURED_GRAPHS', [0])
+    assert parallel.any_rank_captured_graphs() is False
+    monkeypatch.setattr(parallel, '_CAPTURED_GRAPHS', [2])
+    assert parallel.any_rank_captured_graphs() is True
 
 
 def test_user_sharded_lightgcn_row_restricted_layers_world2():

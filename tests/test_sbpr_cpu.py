@@ -1,8 +1,8 @@
 """SBPR drop-in (f-4 sibling model: model/ranking/SBPR.py mirror) on the CPU.
 
-(1) the item sets and the minibatch sampler against the UNMODIFIED reference class in the same process (TensorFlow
-    stubbed: `initModel` and `next_batch` never touch it): same PositiveSet / FPSet, same (u, i, k, j, S_uk) batches
-    from the same `random` state, same generator state afterwards;
+(1) the item sets and the minibatch sampler against the UNMODIFIED reference class, recorded on the same inputs in
+    tests/golden/sbpr_reference_sampler.json.xz (oracle/gen_golden.py social): same PositiveSet / FPSet, same
+    (u, i, k, j, S_uk) batches from the same `random` state, same generator state afterwards;
     and (portable: no reference checkout needed) against the golden record oracle/gen_golden.py made from the unmodified
     reference class on FilmTrust with its real trust network (tests/golden/sbpr_filmtrust_seed77.npz);
 (2) the numpy path stops where the reference's does (SBPR.py:47, TypeError);
@@ -12,17 +12,15 @@ import contextlib
 import io
 import os
 import random
-import sys
-import types
 
 import numpy as np
 import pytest
 
+from oracle import golden_json
 from qrec_b200.util.config import ModelConf
 from test_bpr_model_cpu import _stub_engine
 from test_tbpr_cpu import _data
 
-REF = '/root/reference'
 CONF = '''ratings=x
 social=x
 ratings.setup=-columns 0 1 2
@@ -86,46 +84,22 @@ def test_sbpr_item_sets_and_numpy_path_error(golden_bpr, monkeypatch, tmp_path):
         assert (w == 0 and len(m.FPSet[user]) == 0) or m.FPSet[user][id2item[k]] == w
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='reference checkout not mounted')
 def test_sbpr_sampler_equals_unmodified_reference_class(golden_bpr, monkeypatch, tmp_path):
     calls = []
     _stub_engine(monkeypatch, calls)
     monkeypatch.chdir(tmp_path)
     m, train, test, rel = _model(golden_bpr)
-    before = set(sys.modules)
-    tf = types.ModuleType('tensorflow')
-    for name, mod in (('tensorflow', tf), ('mkl', types.ModuleType('mkl'))):
-        sys.modules.setdefault(name, mod)
-    sys.path.insert(0, REF)
-    try:
-        import importlib
-        R = importlib.import_module('model.ranking.SBPR').SBPR
-        RConf = importlib.import_module('util.config').ModelConf
-        conf_file = tmp_path / 'sbpr.conf'
-        conf_file.write_text(CONF)
-        np.random.seed(1)
-        ref = R(RConf(str(conf_file)), [list(r) for r in train], [list(r) for r in test], [list(r) for r in rel])
-        with contextlib.redirect_stdout(io.StringIO()):
-            ref.readConfiguration()
-            ref.initModel()
-        ref.batch_size = 700
-        assert {u: dict(v) for u, v in ref.PositiveSet.items() if v} == {u: dict(v) for u, v in m.PositiveSet.items() if v}
-        assert {u: dict(v) for u, v in ref.FPSet.items() if v} == {u: dict(v) for u, v in m.FPSet.items() if v}
-        for u in ref.FPSet:
-            assert list(ref.FPSet[u].keys()) == list(m.FPSet[u].keys())         # `choice(list(keys))` depends on the order
-        random.seed(77)
-        ref_batches = [tuple(list(x) for x in b) for b in ref.next_batch()]
-        ref_state = random.getstate()
-    finally:
-        sys.path.remove(REF)
-        for k in set(sys.modules) - before:
-            del sys.modules[k]
+    ref = golden_json.load(os.path.join(os.path.dirname(__file__), 'golden', 'sbpr_reference_sampler.json.xz'))
+    assert ref['positive'] == {u: dict(v) for u, v in m.PositiveSet.items() if v}
+    assert {u: v for u, v in ref['fp'].items() if v} == {u: dict(v) for u, v in m.FPSet.items() if v}
+    for u in ref['fp']:
+        assert list(ref['fp'][u].keys()) == list(m.FPSet[u].keys())          # `choice(list(keys))` depends on the order
     random.seed(77)
     m.batch_size = 700
     ours = [tuple(list(x) for x in b) for b in m.next_batch()]
-    assert random.getstate() == ref_state
-    assert len(ours) == len(ref_batches) == 5
-    for a, b in zip(ours, ref_batches):
+    assert random.getstate() == ref['state']
+    assert len(ours) == len(ref['batches']) == 5
+    for a, b in zip(ours, ref['batches']):
         assert a == b
 
 

@@ -3,24 +3,23 @@ kernels are replaced by the pinned oracle, so what is checked is the HOST side t
 strengths, the per-epoch strong / weak / joint item sets, the preference chains and their draw order from Python's
 `random`, the per-user regulariser quirk of the loss, the learning-rate bookkeeping.
 
-(1) differential against the UNMODIFIED reference class run in the same process (only where /root/reference is
-    mounted: the joint set is iterated in Python set order, which depends on the interpreter's string-hash seed, so
-    a recorded golden stream would not be portable -- a same-process differential is);
+(1) differential against the UNMODIFIED reference class, recorded under a fixed string-hash seed (the joint set is
+    iterated in Python set order, which depends on it) and replayed under the same seed;
 (2) self-consistency that also runs on the GPU box's CPU suite."""
 import contextlib
 import io
 import os
 import random
+import subprocess
 import sys
-import types
 
 import numpy as np
 import pytest
 
+from conftest import GOLDEN, ROOT
 from qrec_b200.util.config import ModelConf
 from test_bpr_model_cpu import _stub_engine
 
-REF = '/root/reference'
 CONF = '''ratings=x
 social=x
 ratings.setup=-columns 0 1 2
@@ -117,42 +116,33 @@ def test_tbpr_host_logic_self_consistency(golden_bpr, monkeypatch, tmp_path):
     assert len(seen['rowptr']) == m.num_users + 1 and seen['rowptr'][-1] == seen['n'] and np.all(np.diff(seen['rowptr']) >= 0)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='reference checkout not mounted')
-def test_tbpr_equals_unmodified_reference_class(golden_bpr, monkeypatch, tmp_path):
-    """Same seeds, same process: epoch losses, learning rates, theta, the final tables and the ranking measures of
-    the drop-in equal those of the reference's TBPR (numpy path) -- K1 being the oracle here."""
+def _record_dropin(path):
+    """The drop-in's side of test_tbpr_equals_unmodified_reference_class, run in a child interpreter."""
     from qrec_b200.model.ranking.TBPR import TBPR
-    train, test, rel = _data(golden_bpr)
-    # ---- the reference, under a private import context
-    before = set(sys.modules)
-    for name in ('tensorflow', 'mkl'):
-        sys.modules.setdefault(name, types.ModuleType(name))
-    sys.path.insert(0, REF)
-    try:
-        import importlib
-        R = importlib.import_module('model.ranking.TBPR').TBPR
-        RConf = importlib.import_module('util.config').ModelConf
-        conf_file = tmp_path / 'tbpr.conf'
-        conf_file.write_text(CONF)
-        monkeypatch.chdir(tmp_path)
-        random.seed(11); np.random.seed(11)
-        ref = R(RConf(str(conf_file)), [list(r) for r in train], [list(r) for r in test], [list(r) for r in rel])
-        ref_losses = []
-        orig = R.isConverged
-        R.isConverged = lambda self, epoch: (ref_losses.append((self.loss, self.lRate)), orig(self, epoch))[1]
-        with contextlib.redirect_stdout(io.StringIO()):
-            ref_measure = ref.execute()
-    finally:
-        sys.path.remove(REF)
-        for k in set(sys.modules) - before:
-            del sys.modules[k]
-    # ---- the drop-in
-    calls = []
-    _stub_engine(monkeypatch, calls)
-    m, losses, measure = _run(TBPR, train, test, rel, CONF)
-    assert m.theta == ref.theta and m.t_s == ref.t_s and m.t_w == ref.t_w
-    assert [l[1] for l in losses] == [l[1] for l in ref_losses]
-    np.testing.assert_allclose([l[0] for l in losses], [l[0] for l in ref_losses], rtol=1e-12)
-    np.testing.assert_allclose(m.P, ref.P, rtol=1e-12, atol=1e-15)
-    np.testing.assert_allclose(m.Q, ref.Q, rtol=1e-12, atol=1e-15)
-    assert [x.strip() for x in measure] == [x.strip() for x in ref_measure]
+    train, test, rel = _data(np.load(os.path.join(GOLDEN, 'bpr_filmtrust_seed0.npz')))
+    with pytest.MonkeyPatch.context() as mp:
+        _stub_engine(mp, [])
+        m, losses, measure = _run(TBPR, train, test, rel, CONF)
+    np.savez(path, theta=m.theta, t_s=m.t_s, t_w=m.t_w, loss=[l[0] for l in losses], lrate=[l[1] for l in losses],
+             P=m.P, Q=m.Q, measure=[x.strip() for x in measure])
+
+
+def test_tbpr_equals_unmodified_reference_class(tmp_path):
+    """Same seeds: epoch losses, learning rates, theta, the final tables and the ranking measures of the drop-in equal
+    those of the reference's TBPR (numpy path), recorded on the same inputs in tests/golden/tbpr_reference_hashseed0.npz
+    -- K1 being the oracle here.  The joint item set is iterated in Python set order, which follows the string-hash
+    seed, so the drop-in runs in a child interpreter under PYTHONHASHSEED=0, the seed the record was made under."""
+    out = tmp_path / 'dropin.npz'
+    code = 'import sys; sys.path[:0] = sys.argv[1:3]; import test_tbpr_cpu; test_tbpr_cpu._record_dropin(sys.argv[3])'
+    run = subprocess.run([sys.executable, '-c', code, ROOT, os.path.dirname(__file__), str(out)], cwd=tmp_path,
+                         env=dict(os.environ, PYTHONHASHSEED='0'), capture_output=True, text=True, timeout=600)
+    assert run.returncode == 0, run.stderr[-3000:]
+    m, ref = np.load(out), np.load(os.path.join(GOLDEN, 'tbpr_reference_hashseed0.npz'))
+    assert m['theta'] == ref['theta'] and m['t_s'] == ref['t_s'] and m['t_w'] == ref['t_w']
+    assert m['lrate'].tolist() == ref['lrate'].tolist()
+    np.testing.assert_allclose(m['loss'], ref['loss'], rtol=1e-12)
+    # the record holds every 5th row of each table whole and the |.|-sum of every row
+    for name in ('P', 'Q'):
+        np.testing.assert_allclose(m[name][ref['rows']], ref[name + '_rows'], rtol=1e-12, atol=1e-15)
+        np.testing.assert_allclose(np.abs(m[name]).sum(1), ref[name + '_abs_row_sums'], rtol=1e-12)
+    assert m['measure'].tolist() == ref['measure'].tolist()
